@@ -307,6 +307,30 @@ def c5_problems(cabi, indices):
     return probs
 
 
+DUMP_BUDGET = 64 << 20  # bytes of .npy data that --dump-outputs may write in all
+
+
+def dump_outputs(out_dir, passes):
+    """What a caller of the timed path receives, per problem of the last timed step: model, inlier mask and RANSAC stats of
+    every pass, as DIR/<pass>_<field>.npy (float64; the masks as float32 0/1).  When the masks of all problems would exceed
+    DUMP_BUDGET, a fixed, seeded sample of the problems is written; <pass>_index.npy holds the problem indices written."""
+    os.makedirs(out_dir, exist_ok=True)
+    count = len(next(iter(passes.values())))
+    per_problem = sum(4 * len(r[0]["inliers"]) + 8 * (len(r[0]["model"].ravel()) + len(r[0]["stats"]) + 1)
+                      for r in passes.values())
+    keep = min(count, (DUMP_BUDGET - (1 << 16)) // per_problem)  # 64 KiB left for the .npy headers
+    index = np.arange(count) if keep == count else np.sort(np.random.default_rng(0).choice(count, keep, replace=False))
+    for name, results in passes.items():
+        rows = [results[i] for i in index]
+        arrays = {"index": index.astype(np.float64),
+                  "model": np.stack([np.asarray(r["model"], dtype=np.float64) for r in rows]),
+                  "inliers": np.stack([np.asarray(r["inliers"], dtype=np.float32) for r in rows])}
+        for key in rows[0]["stats"]:
+            arrays["stats_" + key] = np.array([r["stats"][key] for r in rows], dtype=np.float64)
+        for field, a in arrays.items():
+            np.save(os.path.join(out_dir, f"{name}_{field}.npy"), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -322,7 +346,11 @@ def main():
                     help="headline only: skip the configs 1/3/4 batches, the single calls and the config-5 strong-scaling pass")
     ap.add_argument("--c5", type=int, default=4096, help="problems of the config-5 batch (sharded over the ranks)")
     ap.add_argument("--quick", action="store_true", help="small extras (smoke test of the bench itself)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the results of the last timed step of the headline (resident) and e2e passes as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 0)
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -396,6 +424,8 @@ def main():
     barrier()
     t_e2e, c_e2e, last = timed(host_probs, args.steps, gather=True)
     barrier()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"resident": last_value, "e2e": last})
     # roofline pass: the same workload with ONE lock-step group in flight, so that the CUDA-event duration of the scoring
     # kernel is not inflated by kernels of other groups sharing the GPU (still live, still on the engine's stream)
     streams_saved = args.streams

@@ -3,9 +3,30 @@ solvers/relpose_8pt.cc:52-95) — the device kernel is not built yet (DESIGN.md 
 the ground truth on noise-free data, exactly 8 points and over-determined, (b) returns a matrix with singular values
 (s, s, 0), and (c) equals the reference's own source file run on mini-Eigen bit for bit (logic pin; the symmetric
 eigen-solver is iterative in Eigen, so parity with a real PoseLib build is to tolerance by construction)."""
+import os
+import sys
+
 import numpy as np
 import plo_py as P
 import pytest
+
+sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden"))
+from ref_store import RefStore  # noqa: E402
+
+REF = RefStore("ref_8pt", P.ref2_available())  # the reference's results, stored in tests/golden/ref_8pt/
+
+
+@pytest.fixture(autouse=True, scope="module")
+def _save_store():
+    yield
+    REF.save()
+
+
+@pytest.fixture(autouse=True)
+def _store_key(request):
+    REF.begin(request.node)
+    yield
+    REF.end()
 
 
 def _scene(n, seed, noise=0.0):
@@ -42,12 +63,16 @@ def test_essential_matrix_8pt_recovers_ground_truth(n):
         assert min(np.abs(Rk - R).max() + np.abs(p[4:] - t).max() for Rk, p in zip(Rs, poses)) < 1e-8
 
 
-@pytest.mark.skipif(not P.ref2_available(), reason="oracle/_ref/libplref2.so not built (no /root/reference here)")
+def _reference_8pt(x1, x2):
+    with P.reference_sources():
+        return P.essential_matrix_8pt(x1, x2), P.relpose_8pt(x1, x2)
+
+
 def test_8pt_equals_the_reference_source_on_mini_eigen():
+    """The reference's side: oracle/_ref/libplref2.so, or without it its results stored in tests/golden/ref_8pt/."""
     for n in (8, 9, 12, 50, 300):
         for seed in range(30):
             x1, x2, _, _ = _scene(n, 1000 * n + seed, noise=0.002 if seed % 2 else 0.0)
             a, pa = P.essential_matrix_8pt(x1, x2), P.relpose_8pt(x1, x2)
-            with P.reference_sources():
-                b, pb = P.essential_matrix_8pt(x1, x2), P.relpose_8pt(x1, x2)
+            b, pb = REF(lambda: _reference_8pt(x1, x2))
             assert np.array_equal(a, b) and pa.shape == pb.shape and np.array_equal(pa, pb), (n, seed)

@@ -1,9 +1,13 @@
-"""CPU-only, needs oracle/_ref/libplref.so (built here from /root/reference by `make -C oracle ref`): the parts of the
+"""CPU-only: the parts of the
 UNMODIFIED reference that compile without Eigen — robust/sampling.cc and the loop templates of robust/ransac_impl.h —
 pin (1) the sampler of the oracle AND of the engine bit for bit, (2) the dynamic-iteration arithmetic, (3) the
 control flow of the oracle's ransac<> / score_models<> restatement: the reference's loop drives the oracle's estimators
-and must arrive at exactly the oracle loop's result."""
+and must arrive at exactly the oracle loop's result.
+The reference's side is oracle/_ref/libplref.so (`make -C oracle ref`, where the reference's sources are) or, without
+it, that library's results stored in tests/golden/ref_pins/ (tests/golden/ref_store.py)."""
 import math
+import os
+import sys
 
 import numpy as np
 import plo_py as P
@@ -12,30 +16,46 @@ import pytest
 from poselib_b200 import cabi
 from poselib_b200 import problem_generator as G
 
-pytestmark = pytest.mark.skipif(not P.ref_available(), reason="oracle/_ref not built (no /root/reference on this box)")
+sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden"))
+from ref_store import RefStore  # noqa: E402
+
+REF = RefStore("ref_pins", P.ref_available())  # the reference's results, stored in tests/golden/ref_pins/
+
+
+@pytest.fixture(autouse=True, scope="module")
+def _save_store():
+    yield
+    REF.save()
+
+
+@pytest.fixture(autouse=True)
+def _store_key(request):
+    REF.begin(request.node)
+    yield
+    REF.end()
 
 
 def test_random_int_stream_and_known_answer():
-    r = P.ref_random_ints(0, 6)
+    r = REF(lambda: P.ref_random_ints(0, 6))
     assert r.tolist() == [2065550767, -1581685260, -2146876081, 1917616620, 1369994395, 1954456298]  # SURVEY App. A.1
     for seed in (0, 1, 99, 2**40 + 3):
-        assert np.array_equal(P.ref_random_ints(seed, 4000), P.random_ints(seed, 4000))
+        assert REF.same(lambda: P.ref_random_ints(seed, 4000), P.random_ints(seed, 4000))
 
 
 @pytest.mark.parametrize("n,k", [(10000, 5), (200, 3), (5000, 7), (20000, 4), (7, 7), (6, 5), (33, 4)])
 @pytest.mark.parametrize("seed", [0, 7, 2**33 + 1])
 def test_reference_sampler_pins_oracle_and_engine(n, k, seed):
-    ref = P.ref_sample_table(n, k, P.RansacOpt(seed=seed), 4000)
-    assert np.array_equal(ref, P.sample_table(n, k, P.RansacOpt(seed=seed), 4000))
-    assert np.array_equal(ref, cabi.host_sample_table(n, k, cabi.RansacOpt(seed=seed), 4000))
+    oracle = P.sample_table(n, k, P.RansacOpt(seed=seed), 4000)
+    assert REF.same(lambda: P.ref_sample_table(n, k, P.RansacOpt(seed=seed), 4000), oracle)
+    assert np.array_equal(oracle, cabi.host_sample_table(n, k, cabi.RansacOpt(seed=seed), 4000))
 
 
 @pytest.mark.parametrize("n,k,budget", [(5000, 7, 100000), (400, 5, 300), (50, 4, 40), (64, 3, 100000), (9, 4, 5)])
 def test_reference_prosac_sampler_pins_oracle_and_engine(n, k, budget):
     kw = dict(seed=5, progressive_sampling=True, max_prosac_iterations=budget)
-    ref = P.ref_sample_table(n, k, P.RansacOpt(**kw), 3000)
-    assert np.array_equal(ref, P.sample_table(n, k, P.RansacOpt(**kw), 3000))
-    assert np.array_equal(ref, cabi.host_sample_table(n, k, cabi.RansacOpt(**kw), 3000))
+    oracle = P.sample_table(n, k, P.RansacOpt(**kw), 3000)
+    assert REF.same(lambda: P.ref_sample_table(n, k, P.RansacOpt(**kw), 3000), oracle)
+    assert np.array_equal(oracle, cabi.host_sample_table(n, k, cabi.RansacOpt(**kw), 3000))
 
 
 def test_reference_iteration_arithmetic_pins_oracle_and_engine():
@@ -44,10 +64,10 @@ def test_reference_iteration_arithmetic_pins_oracle_and_engine():
         nd = int(rng.integers(1, 30000))
         ni = int(rng.integers(0, nd + 1))
         k = int(rng.choice([0, 3, 4, 5, 7]))
-        assert P.ref_all_inlier_sample_probability(ni, nd, k) == P.all_inlier_sample_probability(ni, nd, k)
+        assert REF(lambda: P.ref_all_inlier_sample_probability(ni, nd, k)) == P.all_inlier_sample_probability(ni, nd, k)
         sp = float(rng.choice([0.99, 0.9999]))
         mult, mn, mx = float(rng.choice([1.0, 3.0])), int(rng.integers(0, 2000)), int(rng.integers(1, 200000))
-        ref = P.ref_compute_dynamic_max_iter(ni, nd, max(k, 1), math.log(1 - sp), mult, mn, mx)
+        ref = REF(lambda: P.ref_compute_dynamic_max_iter(ni, nd, max(k, 1), math.log(1 - sp), mult, mn, mx))
         assert ref == P.compute_dynamic_max_iter(ni, nd, max(k, 1), math.log(1 - sp), mult, mn, mx)
         if nd >= max(k, 1):
             assert ref == cabi.host_dynamic_max_iter(ni, nd, max(k, 1), sp, mult, mn, mx)
@@ -57,8 +77,8 @@ def test_reference_loop_with_the_mock_estimator_of_the_reference_tests():
     # tests/ransac_test.cc:71-122: exact stop iterations of ransac<MockEstimator, int>
     for nd, k, inl, kw in [(100, 5, 80, {}), (100, 5, 80, dict(min_iterations=50, max_iterations=1000)),
                            (100, 7, 10, dict(min_iterations=10, max_iterations=333)), (10, 5, 10, {}), (4, 5, 4, {})]:
-        r, o = P.ref_ransac_mock(nd, k, inl, P.RansacOpt(**kw)), P.ransac_mock(nd, k, inl, P.RansacOpt(**kw))
-        assert r.as_dict() == o.as_dict()
+        r, o = REF(lambda: P.ref_ransac_mock(nd, k, inl, P.RansacOpt(**kw)).as_dict()), P.ransac_mock(nd, k, inl, P.RansacOpt(**kw))
+        assert r == o.as_dict()
 
 
 CASES = [
@@ -87,11 +107,15 @@ def test_reference_loop_drives_oracle_estimators_to_the_oracle_loop_result(kind,
         else:
             init = np.eye(3) + 0.01
     rfc = kind == "fundamental"
-    r = P.ref_ransac(kind, a, b, P.RansacOpt(**kw), me / G.FOCAL, init=init, rfc=rfc)
+    r = REF(lambda: P.ref_ransac(kind, a, b, P.RansacOpt(**kw), me / G.FOCAL, init=init, rfc=rfc))
     o = P.ransac(kind, a, b, P.RansacOpt(**kw), me / G.FOCAL, init=init, rfc=rfc)
     assert r["stats"] == o["stats"]
     assert np.array_equal(r["inliers"], o["inliers"])
     assert np.array_equal(np.asarray(r["model"]), np.asarray(o["model"]), equal_nan=True)
+
+
+def _roots(n, roots):
+    return n, roots[:max(n, 0)]
 
 
 def test_reference_univariate_solvers_pin_the_oracle_bitwise():
@@ -105,10 +129,8 @@ def test_reference_univariate_solvers_pin_the_oracle_bitwise():
             c = b * b / (4 * a)            # double root
         for name, args, k in (("solve_quadratic_real", (a, b, c), 2), ("solve_cubic_single_real", (a, b, c), 1),
                               ("solve_cubic_real", (a, b, c), 3)):
-            nr, rr = getattr(P, name)(*args, ref=True)
             no, ro = getattr(P, name)(*args)
-            assert nr == no, (name, args)
-            assert np.array_equal(rr[:max(nr, 0)], ro[:max(no, 0)], equal_nan=True), (name, args, rr, ro)
+            assert REF.same(lambda: _roots(*getattr(P, name)(*args, ref=True)), _roots(no, ro)), (name, args, no, ro)
 
 
 def test_reference_sturm_root_isolation_pins_the_oracle_bitwise():
@@ -135,9 +157,8 @@ def test_reference_sturm_root_isolation_pins_the_oracle_bitwise():
     for c in polys:
         c = np.ascontiguousarray(c, dtype=np.float64)
         assert len(c) == 11
-        r, o = P.ref_bisect_sturm10(c), P.bisect_sturm10(c)
-        assert len(r) == len(o), (c, r, o)
-        assert np.array_equal(r, o, equal_nan=True), (c, r, o)
+        o = P.bisect_sturm10(c)
+        assert REF.same(lambda: P.ref_bisect_sturm10(c), o), (c, o)
         exact += 1
     assert exact == len(polys)
 
@@ -149,9 +170,7 @@ def test_reference_p3p_scalar_helpers_pin_the_oracle_bitwise():
         b, c = rng.normal(0, 3, 2)
         if i % 5 == 0:
             c = b * b / 4 + rng.choice([0.0, 1e-13, -1e-13, 5e-13])   # around the THRESHOLD branches
-        okr, rr = P.p3p_root2real(b, c, ref=True)
-        oko, ro = P.p3p_root2real(b, c)
-        assert okr == oko and np.array_equal(rr, ro, equal_nan=True), (b, c)
+        assert REF.same(lambda: P.p3p_root2real(b, c, ref=True), P.p3p_root2real(b, c)), (b, c)
     for _ in range(2000):
         # a consistent instance: three unit bearings, true depths perturbed as the solver's initial estimate would be
         x = rng.normal(size=(3, 3))
@@ -161,9 +180,8 @@ def test_reference_p3p_scalar_helpers_pin_the_oracle_bitwise():
         a12, a13, a23 = (np.sum((X[0] - X[1]) ** 2), np.sum((X[0] - X[2]) ** 2), np.sum((X[1] - X[2]) ** 2))
         b12, b13, b23 = x[0] @ x[1], x[0] @ x[2], x[1] @ x[2]
         l0 = lam * (1 + rng.normal(0, 1e-3, 3))
-        rr = P.p3p_refine_lambda(l0, a12, a13, a23, b12, b13, b23, ref=True)
         ro = P.p3p_refine_lambda(l0, a12, a13, a23, b12, b13, b23)
-        assert np.array_equal(rr, ro, equal_nan=True)
+        assert REF.same(lambda: P.p3p_refine_lambda(l0, a12, a13, a23, b12, b13, b23, ref=True), ro)
 
 
 @pytest.mark.parametrize("kind", ["fundamental", "homography"])
@@ -186,7 +204,7 @@ def test_reference_scorers_and_masks_pin_the_oracle_bitwise(kind):
             models = [gt, gt + rng.normal(0, 1e-3, (3, 3)), rng.normal(size=(3, 3)), np.zeros((3, 3)),
                       np.outer(rng.normal(size=3), rng.normal(size=3)), np.eye(3)]
             for M in models:
-                sr, cr, mr = P.ref_score(kind, M, x1, x2, thr * thr, want_inliers=True)
+                sr, cr, mr = REF(lambda: P.ref_score(kind, M, x1, x2, thr * thr, want_inliers=True))
                 so, co = P.score(kind, M, x1, x2, thr * thr)
                 mo = P.inliers(kind, M, x1, x2, thr * thr)
                 assert cr == co
@@ -206,7 +224,7 @@ def test_reference_real_focal_check_pins_the_oracle():
             F = np.diag([1 / f2, 1 / f2, 1.0]) @ E @ np.diag([1 / f1, 1 / f1, 1.0]) + rng.normal(0, 1e-4, (3, 3)) * (i % 2)
         else:
             F = rng.normal(size=(3, 3))
-        assert P.ref_calculate_RFC(F) == bool(P.calculate_RFC(F))
+        assert REF(lambda: P.ref_calculate_RFC(F)) == bool(P.calculate_RFC(F))
         agree += 1
     assert agree == 3000
 
@@ -228,17 +246,15 @@ def test_reference_camera_scalar_code_pins_the_oracle_bitwise():
     for _ in range(3000):
         k1, k2, rd = rng.normal(0, 0.2), rng.normal(0, 0.05), abs(rng.normal(0, 0.6))
         for two in (0, 1):
-            assert P.undistort_poly(k1, k2, two, rd, ref=True) == P.undistort_poly(k1, k2, two, rd)
+            assert REF.same(lambda: P.undistort_poly(k1, k2, two, rd, ref=True), P.undistort_poly(k1, k2, two, rd))
         d4, x2 = rng.normal(0, [0.3, 0.2, 1e-3, 1e-3]), rng.normal(0, 0.5, 2)
-        assert np.array_equal(P.opencv_distortion(d4, x2, ref=True), P.opencv_distortion(d4, x2))
-        (xr, jr), (xo, jo) = P.opencv_distortion(d4, x2, True, ref=True), P.opencv_distortion(d4, x2, True)
-        assert np.array_equal(xr, xo) and np.array_equal(jr, jo)
+        assert REF.same(lambda: P.opencv_distortion(d4, x2, ref=True), P.opencv_distortion(d4, x2))
+        assert REF.same(lambda: P.opencv_distortion(d4, x2, True, ref=True), P.opencv_distortion(d4, x2, True))
     X = np.c_[rng.uniform(-0.6, 0.6, (500, 2)), np.ones(500)] * rng.uniform(0.5, 9.0, (500, 1))
     for cam in REF_CAMERAS:
-        assert P.ref_camera_focal(cam) == P.camera_focal(cam)
-        assert np.array_equal(P.camera_rescale(cam, 1.0 / 1234.5, ref=True), P.camera_rescale(cam, 1.0 / 1234.5))
+        assert REF.same(lambda: P.ref_camera_focal(cam), P.camera_focal(cam))
+        assert REF.same(lambda: P.camera_rescale(cam, 1.0 / 1234.5, ref=True), P.camera_rescale(cam, 1.0 / 1234.5))
         xp_jac, J, xp = P.camera_project_with_jac(cam, X)
-        assert np.array_equal(P.ref_camera_project(cam, X), xp)
+        assert REF.same(lambda: P.ref_camera_project(cam, X), xp)
         if cam[0] in ("PINHOLE", "SIMPLE_PINHOLE"):
-            rxp, rJ = P.ref_camera_project(cam, X, with_jac=True)
-            assert np.array_equal(rxp, xp_jac) and np.array_equal(rJ, J)
+            assert REF.same(lambda: P.ref_camera_project(cam, X, with_jac=True), (xp_jac, J))

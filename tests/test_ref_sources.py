@@ -1,4 +1,4 @@
-"""CPU-only, needs oracle/_ref/libplref2.so (`make -C oracle ref2`, built here from /root/reference): the reference's
+"""CPU-only: the reference's
 OWN sources for the whole hot path — robust.cc, robust/ransac.cc + ransac_impl.h, robust/estimators/*.cc,
 robust/bundle.cc + optim/*.h, robust/utils.cc, solvers/{p3p,relpose_5pt,relpose_7pt,homography_4pt}.cc,
 misc/{essential,camera_models,univariate}.cc — compiled UNMODIFIED on top of mini-Eigen (oracle/ref/mini), which
@@ -25,14 +25,36 @@ Result of the comparison (asserted below):
     reference's sources on the whole path, degenerate inputs included (last four tests of this file).
   * FixCameraRelativePoseRefiner (tangent Sampson): the oracle models Vector4d::norm() with the SSE2 packet order
     (a0²+a2²)+(a1²+a3²) in that one place; mini-Eigen sums left to right.  Agreement 1e-9.
+The reference's side is oracle/_ref/libplref2.so (`make -C oracle ref2`, where the reference's sources are) or, without
+it, that library's results stored in tests/golden/ref_sources/ (tests/golden/ref_store.py).  The tests that need
+the reference's source text itself (the operation-order table) or its alternative build run only where it is.
 """
+import os
+import sys
+
 import numpy as np
 import plo_py as P
 import pytest
 
 from poselib_b200 import problem_generator as G
 
-pytestmark = pytest.mark.skipif(not P.ref2_available(), reason="oracle/_ref/libplref2.so not built (no /root/reference here)")
+sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden"))
+from ref_store import RefStore  # noqa: E402
+
+REF = RefStore("ref_sources", P.ref2_available())  # the reference's results, stored in tests/golden/ref_sources/
+
+
+@pytest.fixture(autouse=True, scope="module")
+def _save_store():
+    yield
+    REF.save()
+
+
+@pytest.fixture(autouse=True)
+def _store_key(request):
+    REF.begin(request.node, stored="reference_order" not in request.fixturenames)  # runs only with the reference
+    yield
+    REF.end()
 
 CAMT = (G.FOCAL, G.FOCAL, 0.0, 0.0)
 CAMERAS = [("SIMPLE_PINHOLE", [1000.0, 3.0, -4.0]), ("PINHOLE", [1000.0, 1010.0, 3.0, -4.0]),
@@ -42,10 +64,17 @@ CAMERAS = [("SIMPLE_PINHOLE", [1000.0, 3.0, -4.0]), ("PINHOLE", [1000.0, 1010.0,
 
 def both(f):
     """(oracle result, reference-sources result) of the same wrapper call."""
-    a = f()
+    return f(), REF(lambda: reference(f))
+
+
+def reference(f):
     with P.reference_sources():
-        b = f()
-    return a, b
+        return f()
+
+
+def same_as_reference(f):
+    """Bitwise: the oracle's result of the wrapper call equals the reference sources' result."""
+    return REF.same(lambda: reference(f), f())
 
 
 def same(a, b):
@@ -69,8 +98,8 @@ def test_p3p_lambdatwist_is_bit_identical_and_finds_the_pose():
     found = 0
     for s in range(400):
         x, X, R, t = G.minimal_abspose(s)
-        a, b = both(lambda: P.p3p_lambdatwist(x, X))
-        assert a.shape == b.shape and np.array_equal(a, b), s
+        a = P.p3p_lambdatwist(x, X)
+        assert REF.same(lambda: reference(lambda: P.p3p_lambdatwist(x, X)), a), s
         for p in a:
             q = p[:4]
             Rq = np.array([[1 - 2 * (q[2]**2 + q[3]**2), 2 * (q[1] * q[2] - q[0] * q[3]), 2 * (q[1] * q[3] + q[0] * q[2])],
@@ -85,18 +114,15 @@ def test_p3p_lambdatwist_is_bit_identical_and_finds_the_pose():
 def test_p3p_and_homography_4pt_are_bit_identical():
     for s in range(300):
         x, X, _, _ = G.minimal_abspose(s)
-        a, b = both(lambda: P.p3p(x, X))
-        assert a.shape == b.shape and np.array_equal(a, b), s
+        assert same_as_reference(lambda: P.p3p(x, X)), s
         x1, x2, _ = G.minimal_homography(s)
         for cheir in (True, False):
-            (na, Ha), (nb, Hb) = both(lambda: P.homography_4pt(x1, x2, cheir))
-            assert na == nb and np.array_equal(Ha, Hb), s
+            assert same_as_reference(lambda: P.homography_4pt(x1, x2, cheir)), s
     # degenerate input: three collinear points, and a cheirality violation
     x1, x2, _ = G.minimal_homography(0)
     x1c = x1.copy()
     x1c[2] = 0.5 * (x1c[0] + x1c[1])
-    (na, Ha), (nb, Hb) = both(lambda: P.homography_4pt(x1c, x2, False))
-    assert na == nb and np.array_equal(Ha, Hb, equal_nan=True)
+    assert same_as_reference(lambda: P.homography_4pt(x1c, x2, False))
     x2f = x2.copy()
     x2f[3] = -x2f[3]
     (na, _), (nb, _) = both(lambda: P.homography_4pt(x1, x2f, True))
@@ -160,13 +186,11 @@ def test_camera_models_are_bit_identical(cam):
     rng = np.random.default_rng(0)
     X = np.c_[rng.uniform(-0.4, 0.4, (300, 2)), np.ones(300)]
     X /= np.linalg.norm(X, axis=1)[:, None]
-    a, b = both(lambda: P.camera_project_with_jac(cam, X))
-    assert same(a, b)
-    xp = a[2]
-    assert same(*both(lambda: P.camera_unproject_with_jac(cam, xp)))
-    assert same(*both(lambda: P.camera_unproject2(cam, xp)))
-    fa, fb = both(lambda: P.camera_focal(cam))
-    assert fa == fb
+    assert same_as_reference(lambda: P.camera_project_with_jac(cam, X))
+    xp = P.camera_project_with_jac(cam, X)[2]
+    assert same_as_reference(lambda: P.camera_unproject_with_jac(cam, xp))
+    assert same_as_reference(lambda: P.camera_unproject2(cam, xp))
+    assert same_as_reference(lambda: P.camera_focal(cam))
 
 
 # ---- RANSAC and estimate_*, end to end ---------------------------------------------------------------------------
